@@ -69,14 +69,14 @@ def ensure_built() -> str | None:
 
 
 def run(args) -> int:
-    err = ensure_built()
-    if err:
-        return _unavailable(err)
-    sys.path.insert(0, os.path.join(HERE, "_ref"))
     import torch
 
     if not torch.cuda.is_available():
         return _unavailable("no CUDA device visible")
+    err = ensure_built()
+    if err:
+        return _unavailable(err)
+    sys.path.insert(0, os.path.join(HERE, "_ref"))
     local_rank = int(os.environ.get("LOCAL_RANK", os.environ.get("RANK", "0")))
     torch.cuda.set_device(local_rank % torch.cuda.device_count())
     dev = torch.device("cuda", torch.cuda.current_device())

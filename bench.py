@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Headline benchmark (driver contract: see the task brief / DESIGN.md).
+"""Headline benchmark (see DESIGN.md).
 
 Flagship step = BASELINE.json config "4096x4096 linear layer: Allreduce(params)
 -> GEMM fused, loss Allreduce backward": every rank holds a 4096x4096 bf16
@@ -12,6 +12,7 @@ weight and a private batch; one step is, THROUGH THE AUTOGRAD GRAPH,
 
     python bench.py --gpus N --steps K --warmup W            (N>1: under torchrun)
     python bench.py --impl reference ...                      (the unmodified reference, baseline/)
+    python bench.py ... --dump-outputs DIR                    (also write the last timed step's results as .npy)
 
 Prints ONE JSON line on rank 0.  `value` = samples/s over the whole job, timed on the device (CUDA
 events, max over ranks); `e2e` = the same step through the public API including per-step H2D of the
@@ -36,6 +37,7 @@ METRIC = "dp_linear4096_train_samples_per_s"
 IN_F = OUT_F = 4096
 PER_GPU_BATCH = 8192
 POOL = 4  # rotating input batches: 4 x (64 MiB x + 64 MiB t) >> 126 MB L2
+DUMP_SAMPLE = 1 << 22  # weight elements written by --dump-outputs (16 MiB as float32)
 
 
 def linreg_cpu_step_per_s() -> object:
@@ -55,6 +57,20 @@ def linreg_cpu_step_per_s() -> object:
         return {"error": f"{type(exc).__name__}: {exc}"[:200]}
 
 
+def dump_outputs(out_dir: str, loss, weight) -> None:
+    """What the last timed step hands its caller, as float32 .npy files: the global loss and the updated weight.
+    The weight is written as a fixed sample of DUMP_SAMPLE elements (seeded, in flat index order), so two builds
+    run with the same arguments can be compared element for element."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    flat = weight.detach().reshape(-1)
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().reshape(1).cpu().numpy())
+    np.save(os.path.join(out_dir, "weight_sample.npy"), flat[idx.to(flat.device)].float().cpu().numpy())
+
+
 def main() -> int:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -67,6 +83,8 @@ def main() -> int:
     ap.add_argument("--unfused", action="store_true", help="force the unfused Allreduce + GEMM composition")
     ap.add_argument("--plain-sgd", action="store_true", help="weight.grad + separate SGD instead of the optimizer in backward")
     ap.add_argument("--full-sweep", action="store_true", help="1 KiB .. 1 GiB in x4 steps instead of the quick table")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's loss and a fixed sample of the updated weight to DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         sys.path.insert(0, os.path.join(ROOT, "baseline"))
@@ -150,6 +168,10 @@ def main() -> int:
     # which tensor-core / fused kernels really ran in the timed region (launches per step)
     path = {k: (v - table0.get(k, 0)) / args.steps for k, v in dict(_C.kernel_launch_table()).items()
             if v - table0.get(k, 0) > 0}
+    if args.dump_outputs:  # before the end-to-end region trains the same model further
+        if rank == 0:
+            dump_outputs(args.dump_outputs, loss, model.weight)
+        comm.Barrier()
 
     # ---------------- end-to-end region (public API + H2D/D2H every step) ----------------
     pin_x = [torch.randn(B, IN_F, dtype=torch.bfloat16).pin_memory() for _ in range(2)]

