@@ -7,7 +7,8 @@ Gather / Allgather / Scatter / Alltoall / Isend / Irecv / Wait / Send / Recv``,
 reduction constants, ``comm_from_mpi4py`` and
 ``deactivate_cuda_aware_mpi_support`` - every op a differentiable graph node
 whose backward is the adjoint communication.  Added on top: ``Reduce_scatter``
-(the true adjoint of ``Allgather``), fused scale/accumulate epilogues
+(the true adjoint of ``Allgather``), ``Scan`` / ``Exscan`` (prefix reductions across
+ranks), fused scale/accumulate epilogues
 (``AllreduceFused``), ``Barrier`` and the fused Allreduce->GEMM layer in
 :mod:`mpi4torch_b200.ops`.
 
@@ -325,6 +326,25 @@ class MPI_Communicator:
         csrc/extension.cpp:616-631).  Backward: ``Allgather(scale * grad)``; ``accumulate`` receives the
         incoming gradient."""
         return self._comm.Reduce_scatterFused(tensor, op, scatteraxis, numelem, scale, accumulate)
+
+    def Scan(self, tensor: torch.Tensor, op: int) -> torch.Tensor:
+        """Inclusive prefix reduction across ranks (``MPI_Scan``): rank ``r`` receives
+        ``((x_0 op x_1) op x_2) ... op x_r``, folded left to right in ascending rank order.
+
+        Every rank passes the same shape and dtype (no size exchange, as in :meth:`Allreduce`);
+        the ops and dtypes are those of :meth:`Allreduce`.  16-bit floats fold in fp32 and are
+        rounded once.  The fold order is part of the contract: every backend and algorithm gives
+        the same bits.  Only ``MPI_SUM`` has a backward: the reverse inclusive scan of the gradient
+        (rank ``r`` receives the sum of the gradients of ranks ``r .. P-1``)."""
+        return self._comm.Scan(tensor, op)
+
+    def Exscan(self, tensor: torch.Tensor, op: int) -> torch.Tensor:
+        """Exclusive prefix reduction across ranks (``MPI_Exscan``): rank ``r > 0`` receives the
+        fold of ``x_0 .. x_{r-1}`` in ascending rank order, as in :meth:`Scan`.  Rank 0's result
+        is zero-filled (MPI leaves it undefined; :meth:`Reduce_` zero-fills non-root results the
+        same way).  Only ``MPI_SUM`` has a backward: the reverse exclusive scan of the gradient
+        (rank ``P-1`` receives zeros)."""
+        return self._comm.Exscan(tensor, op)
 
     def assume_uniform_sizes(self, on: bool = True) -> None:
         """Promise that every rank passes identically shaped tensors and the same ``numelem`` to

@@ -32,6 +32,7 @@ _SOURCES = [
     "runtime/cuda_backend.cpp",
     "runtime/world.cpp",
     "kernels/allreduce.cu",
+    "kernels/scan.cu",
     "kernels/slab.cu",
     "kernels/slab_push.cu",
     "kernels/rooted.cu",

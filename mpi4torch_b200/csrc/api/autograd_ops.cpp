@@ -8,6 +8,8 @@
 //                                                         intended reduce-scatter, not the
 //                                                         reference's literal-root-1 loop)
 //   Alltoall(g,s)    <-> Alltoall(s,g)                  (:903-915)
+//   Scan(SUM)        <-> reverse Scan(SUM)              (prefix sums from rank P-1 downwards)
+//   Exscan(SUM)      <-> reverse Exscan(SUM)
 //   Isend            <-> Irecv, started in WaitBackward (:1173-1218), tag + 10 (:1161)
 //   JoinDummies      :   zero grads to the dummies      (:1013-1022)
 //
@@ -191,6 +193,39 @@ struct MPIReduceScatterBackward : public Function<MPIReduceScatterBackward> {
     Tensor gacc = ctx->saved_data["has_acc"].toBool() ? grads[0] : Tensor();
     return {comm->Allgather(g, ctx->saved_data["axis"].toInt()), Tensor(), Tensor(), Tensor(), Tensor(), Tensor(), Tensor(),
             gacc};
+  }
+};
+
+// ------------------------------------------------------------ Scan / Exscan
+// d out_q / d x_p = 1 for every p at or before q in the fold, so the adjoint sums the gradients of the ranks at or
+// after p: the same scan in the opposite direction (exclusive stays exclusive).
+struct MPIScanSumBackward : public Function<MPIScanSumBackward> {
+  static Tensor forward(AutogradContext* ctx, const Tensor& input, c10::intrusive_ptr<Communicator> comm, int64_t op,
+                        bool reverse) {
+    ctx->saved_data["comm"] = comm;
+    ctx->saved_data["op"] = op;
+    ctx->saved_data["reverse"] = reverse;
+    return comm->raw_scan(input, op, /*exclusive=*/false, reverse);
+  }
+  static variable_list backward(AutogradContext* ctx, variable_list grads) {
+    if (ctx->saved_data["op"].toInt() != kOpSum) unimplemented_backward();
+    auto comm = comm_from(ctx);
+    return {comm->scan_op(grads[0], kOpSum, false, !ctx->saved_data["reverse"].toBool()), Tensor(), Tensor(), Tensor()};
+  }
+};
+
+struct MPIExscanSumBackward : public Function<MPIExscanSumBackward> {
+  static Tensor forward(AutogradContext* ctx, const Tensor& input, c10::intrusive_ptr<Communicator> comm, int64_t op,
+                        bool reverse) {
+    ctx->saved_data["comm"] = comm;
+    ctx->saved_data["op"] = op;
+    ctx->saved_data["reverse"] = reverse;
+    return comm->raw_scan(input, op, /*exclusive=*/true, reverse);
+  }
+  static variable_list backward(AutogradContext* ctx, variable_list grads) {
+    if (ctx->saved_data["op"].toInt() != kOpSum) unimplemented_backward();
+    auto comm = comm_from(ctx);
+    return {comm->scan_op(grads[0], kOpSum, true, !ctx->saved_data["reverse"].toBool()), Tensor(), Tensor(), Tensor()};
   }
 };
 
@@ -426,6 +461,17 @@ Tensor Communicator::Reduce_scatterFused(const Tensor& input, int64_t op, int64_
     return raw_reduce_scatter(input, op, scatteraxis, numelem, scale, true, accumulate);
   return MPIReduceScatterBackward::apply(input, c10::intrusive_ptr<Communicator>::reclaim_copy(this), op, scatteraxis,
                                          numelem, scale, true, accumulate);
+}
+
+Tensor Communicator::Scan(const Tensor& input, int64_t op) { return scan_op(input, op, false, false); }
+
+Tensor Communicator::Exscan(const Tensor& input, int64_t op) { return scan_op(input, op, true, false); }
+
+Tensor Communicator::scan_op(const Tensor& input, int64_t op, bool exclusive, bool reverse) {
+  if (!any_requires_grad({input})) return raw_scan(input, op, exclusive, reverse);
+  auto self = c10::intrusive_ptr<Communicator>::reclaim_copy(this);
+  if (exclusive) return MPIExscanSumBackward::apply(input, self, op, reverse);
+  return MPIScanSumBackward::apply(input, self, op, reverse);
 }
 
 std::vector<Tensor> Communicator::Isend(const Tensor& input, int64_t dest, int64_t tag) {

@@ -82,6 +82,8 @@ TORCH_LIBRARY(mpi4torch_b200, m) {
       .def("Alltoall", &Communicator::Alltoall)
       .def("Reduce_scatter", &Communicator::Reduce_scatter)
       .def("Reduce_scatterFused", &Communicator::Reduce_scatterFused)
+      .def("Scan", &Communicator::Scan)
+      .def("Exscan", &Communicator::Exscan)
       .def("AssumeUniformSizes", &Communicator::AssumeUniformSizes)
       .def("UniformSizes", &Communicator::UniformSizes)
       .def("Isend", &Communicator::Isend)

@@ -313,6 +313,19 @@ void Communicator::raw_reduce_(Tensor& work, int64_t op_, int64_t root) {
   }
 }
 
+Tensor Communicator::raw_scan(const Tensor& input, int64_t op_, bool exclusive, bool reverse) {
+  NvtxRange nvtx_range_(exclusive ? "m4t::Exscan" : "m4t::Scan");
+  const ReduceOp op = to_op(op_);
+  const DType dt = to_dtype(input.scalar_type());
+  check_op_dtype(op, dt);
+  std::lock_guard<std::recursive_mutex> g(world_->mutex());
+  Route r(*world_, cx(), input);
+  Tensor in = r.to_comm(input);
+  Tensor out = at::empty_like(in, at::MemoryFormat::Contiguous);
+  r.be->scan(in.data_ptr(), out.data_ptr(), in.numel(), dt, op, exclusive, reverse, r.stream);
+  return r.from_comm(out);
+}
+
 void Communicator::exchange_meta(const int64_t* mine, int words, int64_t* all) {
   if (uniform_) {  // AssumeUniformSizes: every rank holds the same words, no host round
     for (int64_t p = 0; p < size_; ++p) std::copy(mine, mine + words, all + p * words);

@@ -40,6 +40,12 @@ struct Communicator : torch::CustomClassHolder {
   // Backward: Allgather of (scale * grad); `accumulate` receives the incoming gradient unchanged.
   Tensor Reduce_scatterFused(const Tensor& input, int64_t op, int64_t scatteraxis, int64_t numelem, double scale,
                              const c10::optional<Tensor>& accumulate);
+  // MPI_Scan / MPI_Exscan: the left fold of the inputs of ranks 0..r (Exscan: 0..r-1, zeros on rank 0) in
+  // ascending rank order.  Backward (MPI_SUM only) is the reverse inclusive / exclusive scan of the gradient.
+  Tensor Scan(const Tensor& input, int64_t op);
+  Tensor Exscan(const Tensor& input, int64_t op);
+  // Both directions as one differentiable entry point; `reverse` folds from rank P-1 downwards (the adjoint).
+  Tensor scan_op(const Tensor& input, int64_t op, bool exclusive, bool reverse);
 
   // ---- differentiable non-blocking point-to-point ---------------------------
   std::vector<Tensor> Isend(const Tensor& input, int64_t dest, int64_t tag);
@@ -71,6 +77,7 @@ struct Communicator : torch::CustomClassHolder {
   void raw_allreduce_axpy_(Tensor& param, const Tensor& grad, double scale, int64_t max_blocks = 0);
   void raw_bcast_(Tensor& work, int64_t root);
   void raw_reduce_(Tensor& work, int64_t op, int64_t root);
+  Tensor raw_scan(const Tensor& input, int64_t op, bool exclusive, bool reverse);
   Tensor raw_gather(const Tensor& input, int64_t axis, int64_t root, bool all);
   Tensor raw_scatter(const Tensor& input, int64_t axis, int64_t numelem, int64_t root);
   Tensor raw_alltoall(const Tensor& input, int64_t gatheraxis, int64_t scatteraxis, int64_t numelem);

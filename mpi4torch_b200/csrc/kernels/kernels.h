@@ -54,6 +54,14 @@ void launch_allreduce(const DeviceComm& dc, const void* in, void* out, int64_t n
 void launch_local_epilogue(const void* in, void* out, int64_t n, DType dt, ReduceOp op, const Epilogue& epi,
                            int sm_count, cudaStream_t stream);
 
+// Bytes of staging (per half) a scan of n elements needs with `algo` (ONESHOT or TWOSHOT).
+int64_t scan_stage_bytes(int64_t n, DType dt, ArAlgo algo, int size);
+// out = fold of `in` over the ranks before me in ascending rank order (scan.cu): inclusive (Scan)
+// or exclusive (Exscan, zeros on the first rank of the order); `reverse` folds from rank P-1 down.
+// One launch; the message must fit one staging half (scan_stage_bytes).
+void launch_scan(const DeviceComm& dc, const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive,
+                 bool reverse, ArAlgo algo, int blocks, cudaStream_t stream);
+
 // Broadcast root's private buffer in place (NVLS push when mc_heap, else peer pull).
 void launch_bcast(const DeviceComm& dc, void* buf, int64_t n, DType dt, int root, int blocks,
                   cudaStream_t stream);

@@ -29,6 +29,12 @@ class Backend {
   // In place reduce to root; non-root buffers are zero-filled afterwards
   // (reference csrc/extension.cpp:443-447).
   virtual void reduce(void* buf, int64_t n, DType dt, ReduceOp op, int root, void* stream) = 0;
+  // Prefix reduction across ranks (Scan / Exscan).  out = left fold of `in` over the ranks in
+  // ascending order up to and including me (exclusive: up to the rank before me, zeros on rank 0);
+  // `reverse` folds from rank P-1 downwards instead (the adjoint of a SUM scan).  16-bit floats fold
+  // in fp32 and are rounded once; every backend gives the same bits.
+  virtual void scan(const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive, bool reverse,
+                    void* stream) = 0;
   // Strided box pulls (Gather / Allgather / Scatter / Alltoall).
   virtual void pull(const PullPlan& plan, const void* in, void* out, DType dt, void* stream) = 0;
   // Reduce-scatter along an axis (Allgather's adjoint).

@@ -192,6 +192,55 @@ void CpuBackend::reduce(void* buf, int64_t n, DType dt, ReduceOp op, int root, v
   }
 }
 
+void CpuBackend::scan(const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive, bool reverse, void*) {
+  check_op_dtype(op, dt);
+  const int P = ctl_.size(), r = ctl_.rank();
+  const int64_t es = dtype_size(dt);
+  const size_t bytes = static_cast<size_t>(n * es);
+  if (n == 0) return;
+  if (P == 1) {
+    if (exclusive) {
+      std::memset(out, 0, bytes);
+    } else {
+      const void* srcs[1] = {in};
+      M4T_DISPATCH_DTYPE_OP(dt, op, CpuReduceRange, srcs, 1, out, 0, n, nullptr);
+    }
+    return;
+  }
+  if (static_cast<int64_t>(bytes) > kPieceBytes) {  // cache-sized pieces, as in allreduce
+    const int64_t step = kPieceBytes / es;
+    for (int64_t off = 0; off < n; off += step)
+      scan(static_cast<const char*>(in) + off * es, static_cast<char*>(out) + off * es, std::min(step, n - off), dt, op,
+           exclusive, reverse, nullptr);
+    return;
+  }
+  auto fold_rank = [&](int k) { return reverse ? P - 1 - k : k; };  // rank at position k of the fold
+  const int me = reverse ? P - 1 - r : r;
+  const int par = static_cast<int>(op_seq_++ & 1);
+  const bool two_phase = static_cast<int64_t>(bytes) >= kTwoPhaseBytes;
+  char* mine = stage(par, two_phase ? 2 * bytes : bytes);
+  par_memcpy(mine, in, bytes);
+  ctl_.barrier();
+  const void* srcs[kMaxRanks];
+  for (int k = 0; k < P; ++k) srcs[k] = peer_arena(fold_rank(k), par);
+  if (!two_phase) {
+    const int cnt = exclusive ? me : me + 1;
+    if (cnt == 0) {
+      std::memset(out, 0, bytes);
+      return;
+    }
+    M4T_DISPATCH_DTYPE_OP(dt, op, CpuReduceRange, srcs, cnt, out, 0, n, nullptr);
+    return;
+  }
+  // phase 1: the owner of slice r writes every rank's prefix of it into that rank's result half
+  void* dsts[kMaxRanks];
+  for (int k = 0; k < P; ++k) dsts[k] = const_cast<char*>(static_cast<const char*>(srcs[k])) + bytes;
+  M4T_DISPATCH_DTYPE_OP(dt, op, CpuScanRange, srcs, dsts, P, exclusive, n * r / P, n * (r + 1) / P);
+  ctl_.barrier();
+  // phase 2: my prefixes of all slices are in my own result half
+  par_memcpy(out, mine + bytes, bytes);
+}
+
 void CpuBackend::pull(const PullPlan& plan, const void* in, void* out, DType dt, void*) {
   const int P = ctl_.size(), r = ctl_.rank();
   const int64_t es = dtype_size(dt);

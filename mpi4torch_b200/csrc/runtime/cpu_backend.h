@@ -27,6 +27,10 @@ class CpuBackend final : public Backend {
                  void* stream) override;
   void bcast(void* buf, int64_t n, DType dt, int root, void* stream) override;
   void reduce(void* buf, int64_t n, DType dt, ReduceOp op, int root, void* stream) override;
+  // Scan / Exscan: small messages fold the peers' staged copies in order; from kTwoPhaseBytes the owner of slice p
+  // writes every rank's prefix of slice p into that rank's result half (two barriers)
+  void scan(const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive, bool reverse,
+            void* stream) override;
   void pull(const PullPlan& plan, const void* in, void* out, DType dt, void* stream) override;
   void reduce_pull(const ReducePlan& plan, const void* in, void* out, DType dt, ReduceOp op,
                    const Epilogue& epi, void* stream) override;

@@ -275,6 +275,36 @@ void CudaBackend::reduce(void* buf, int64_t n, DType dt, ReduceOp op, int root, 
     launch_reduce(dc_, static_cast<char*>(buf) + off * es, std::min(max_elems, n - off), dt, op, root, tune_.ar_blocks, s);
 }
 
+void CudaBackend::scan(const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive, bool reverse,
+                       void* stream) {
+  check_device_error();
+  check_op_dtype(op, dt);
+  if (n == 0) return;
+  M4T_CUDA(cudaSetDevice(device_));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int64_t es = dtype_size(dt);
+  if (size() == 1) {
+    if (exclusive) launch_zero(out, n * es, dc_.sm_count, s);
+    else launch_local_epilogue(in, out, n, dt, op, Epilogue{}, dc_.sm_count, s);
+    return;
+  }
+  chain(s);
+  // the Allreduce's choice, with two-shot where it would take NVLS (the switch only returns full reductions, never
+  // prefixes)
+  ArAlgo algo = pick_algo(n * es, dt, op);
+  if (algo == ArAlgo::NVLS) algo = ArAlgo::TWOSHOT;
+  const int blocks = algo == ArAlgo::ONESHOT ? tune_.oneshot_blocks : tune_.ar_blocks;
+  // pieces that fit one staging half: P slots (one-shot) or [in copy | result] (two-shot); multiples of
+  // 128 bytes, so every piece keeps the alignment of the whole tensor
+  const int64_t max_bytes = algo == ArAlgo::ONESHOT ? (dc_.half_bytes / size()) / 128 * 128 - 128
+                                                    : (dc_.half_bytes / 2 - 256) / 128 * 128;
+  const int64_t max_elems = std::max<int64_t>(16, max_bytes / es);
+  for (int64_t off = 0; off < n; off += max_elems)
+    launch_scan(dc_, static_cast<const char*>(in) + off * es, static_cast<char*>(out) + off * es,
+                std::min(max_elems, n - off), dt, op, exclusive, reverse, algo, blocks, s);
+  check_device_error();
+}
+
 namespace {
 int grid_for(int64_t max_elems, int64_t es, int cap) {
   const int64_t vecs = (max_elems * es + 15) / 16;

@@ -49,6 +49,8 @@ class CudaBackend final : public Backend {
                  void* stream) override;
   void bcast(void* buf, int64_t n, DType dt, int root, void* stream) override;
   void reduce(void* buf, int64_t n, DType dt, ReduceOp op, int root, void* stream) override;
+  void scan(const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive, bool reverse,
+            void* stream) override;
   void pull(const PullPlan& plan, const void* in, void* out, DType dt, void* stream) override;
   void reduce_pull(const ReducePlan& plan, const void* in, void* out, DType dt, ReduceOp op,
                    const Epilogue& epi, void* stream) override;

@@ -89,6 +89,53 @@ template <DType DT, ReduceOp OP> struct CpuReduceRange {
   }
 };
 
+// Running fold for Scan / Exscan: dsts[k][i] = combine of srcs[0..k][i] (exclusive: of srcs[0..k-1][i], zero for
+// k = 0) for i in [lo, hi).  Per element this is exactly CpuReduceRange's fold over the first sources, so a rank that
+// folds its own prefix and a slice owner that writes everybody's prefixes produce the same bits.
+template <DType DT, ReduceOp OP> struct CpuScanRange {
+  using E = Elem<DT>;
+  using S = typename E::storage;
+  using A = typename E::acc;
+  using C = Combine<OP, A, E::is_float>;
+
+  static void run_serial(const void* const* srcs, void* const* dsts, int nsrc, bool exclusive, int64_t lo, int64_t hi) {
+    constexpr int kBlock = 512;
+    A buf[kBlock];
+    for (int64_t b0 = lo; b0 < hi; b0 += kBlock) {
+      const int n = static_cast<int>(std::min<int64_t>(kBlock, hi - b0));
+      for (int k = 0; k < nsrc; ++k) {
+        S* d = static_cast<S*>(dsts[k]) + b0;
+        if (exclusive) {
+          if (k == 0) std::memset(d, 0, static_cast<size_t>(n) * sizeof(S));
+          else for (int j = 0; j < n; ++j) d[j] = E::store(buf[j]);
+          if (k == nsrc - 1) break;
+        }
+        const S* sk = static_cast<const S*>(srcs[k]) + b0;
+        if (k == 0) for (int j = 0; j < n; ++j) buf[j] = normalise_single<OP, A>(E::load(sk[j]));
+        else for (int j = 0; j < n; ++j) buf[j] = C::apply(buf[j], E::load(sk[j]));
+        if (!exclusive) for (int j = 0; j < n; ++j) d[j] = E::store(buf[j]);
+      }
+    }
+  }
+
+  static void run(const void* const* srcs, void* const* dsts, int nsrc, bool exclusive, int64_t lo, int64_t hi) {
+    const int64_t n = hi - lo;
+    const int threads = omp_get_max_threads();
+    if (n <= 0) return;
+    if (static_cast<size_t>(n) * sizeof(S) < kParallelBytes || threads <= 1 || omp_in_parallel()) {
+      run_serial(srcs, dsts, nsrc, exclusive, lo, hi);
+      return;
+    }
+    const int64_t per = ((n + threads - 1) / threads + 511) / 512 * 512;
+#pragma omp parallel for schedule(static)
+    for (int t = 0; t < threads; ++t) {
+      const int64_t a = lo + static_cast<int64_t>(t) * per;
+      const int64_t b = std::min(hi, a + per);
+      if (a < b) run_serial(srcs, dsts, nsrc, exclusive, a, b);
+    }
+  }
+};
+
 // dst[i] = acc[i] + src[i]  (phase-2 epilogue of the two-phase allreduce)
 template <DType DT, ReduceOp OP> struct CpuAccumulateCopy {
   static void run(const void* src, const void* acc, void* dst, int64_t lo, int64_t hi) {

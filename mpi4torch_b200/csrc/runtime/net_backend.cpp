@@ -221,6 +221,82 @@ void NetBackend::reduce(void* buf, int64_t n, DType dt, ReduceOp op, int root, v
   M4T_DISPATCH_DTYPE_OP(dt, op, CpuReduceRange, srcs, P, buf, 0, n, nullptr);
 }
 
+void NetBackend::scan(const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive, bool reverse, void*) {
+  check_op_dtype(op, dt);
+  const int P = size(), r = rank();
+  const int64_t es = dtype_size(dt);
+  const size_t bytes = static_cast<size_t>(n * es);
+  if (n == 0) return;
+  if (P == 1) {
+    if (exclusive) {
+      std::memset(out, 0, bytes);
+    } else {
+      const void* srcs[1] = {in};
+      M4T_DISPATCH_DTYPE_OP(dt, op, CpuReduceRange, srcs, 1, out, 0, n, nullptr);
+    }
+    return;
+  }
+  auto fold_rank = [&](int k) { return reverse ? P - 1 - k : k; };  // rank at position k of the fold
+  auto fold_pos = [&](int p) { return reverse ? P - 1 - p : p; };
+  const int me = fold_pos(r);
+  const int64_t tag = link_->next_seq() * 4;
+  NetEngine& eng = link_->engine();
+  const void* srcs[kMaxRanks];
+  std::vector<uint64_t> ops;
+  if (static_cast<int64_t>(bytes) <= kDirectBytes || n < P) {
+    // my vector goes to the ranks after me in the fold; I receive the ones before me and fold them in order
+    NetBuffer& tmp = scratch_[0];
+    grow(tmp, bytes * static_cast<size_t>(me));
+    for (int k = 0; k < me; ++k) {
+      char* slot = tmp.data() + bytes * static_cast<size_t>(k);
+      srcs[k] = slot;
+      ops.push_back(link_->recv(fold_rank(k), kNetColl, tag, slot, bytes));
+    }
+    for (int k = me + 1; k < P; ++k) ops.push_back(link_->send(fold_rank(k), kNetColl, tag, in, bytes));
+    eng.wait_all(ops);
+    srcs[me] = in;
+    const int cnt = exclusive ? me : me + 1;
+    if (cnt == 0) std::memset(out, 0, bytes);
+    else M4T_DISPATCH_DTYPE_OP(dt, op, CpuReduceRange, srcs, cnt, out, 0, n, nullptr);
+    return;
+  }
+  // the owner of slice p receives that slice from every rank, folds it in order and sends rank q its prefix of it:
+  // every rank sends and receives (P-1)/P of the message twice, as in the Allreduce
+  auto lo = [&](int p) { return n * p / P; };
+  const int64_t mylo = lo(r), mylen = lo(r + 1) - lo(r);
+  const size_t slice_bytes = static_cast<size_t>(mylen * es);
+  NetBuffer& tmp = scratch_[0];
+  NetBuffer& res = scratch_[1];
+  grow(tmp, slice_bytes * static_cast<size_t>(P));
+  grow(res, slice_bytes * static_cast<size_t>(P));
+  void* dsts[kMaxRanks];
+  for (int k = 0; k < P; ++k) {
+    const int p = fold_rank(k);
+    dsts[k] = p == r ? static_cast<char*>(out) + mylo * es : res.data() + slice_bytes * static_cast<size_t>(k);
+    if (p == r) {
+      srcs[k] = static_cast<const char*>(in) + mylo * es;
+      continue;
+    }
+    char* slot = tmp.data() + slice_bytes * static_cast<size_t>(k);
+    srcs[k] = slot;
+    ops.push_back(link_->recv(p, kNetColl, tag, slot, slice_bytes));
+  }
+  for (int p = 0; p < P; ++p)
+    if (p != r)
+      ops.push_back(link_->send(p, kNetColl, tag, static_cast<const char*>(in) + lo(p) * es,
+                                static_cast<size_t>((lo(p + 1) - lo(p)) * es)));
+  eng.wait_all(ops);
+  ops.clear();
+  M4T_DISPATCH_DTYPE_OP(dt, op, CpuScanRange, srcs, dsts, P, exclusive, 0, mylen);
+  for (int p = 0; p < P; ++p)
+    if (p != r)
+      ops.push_back(link_->recv(p, kNetColl, tag + 1, static_cast<char*>(out) + lo(p) * es,
+                                static_cast<size_t>((lo(p + 1) - lo(p)) * es)));
+  for (int k = 0; k < P; ++k)
+    if (fold_rank(k) != r) ops.push_back(link_->send(fold_rank(k), kNetColl, tag + 1, dsts[k], slice_bytes));
+  eng.wait_all(ops);
+}
+
 void NetBackend::pull(const PullPlan& plan, const void* in, void* out, DType dt, void*) {
   const int P = size(), r = rank();
   const int64_t es = dtype_size(dt);

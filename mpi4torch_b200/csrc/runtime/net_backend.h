@@ -31,6 +31,10 @@ class NetBackend final : public Backend {
                  void* stream) override;
   void bcast(void* buf, int64_t n, DType dt, int root, void* stream) override;
   void reduce(void* buf, int64_t n, DType dt, ReduceOp op, int root, void* stream) override;
+  // Scan / Exscan  small: every rank receives the contributions of the ranks before it in the fold; large: the owner of
+  //                slice p receives slice p from every rank, folds it in order and returns each rank its prefix
+  void scan(const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive, bool reverse,
+            void* stream) override;
   void pull(const PullPlan& plan, const void* in, void* out, DType dt, void* stream) override;
   void reduce_pull(const ReducePlan& plan, const void* in, void* out, DType dt, ReduceOp op, const Epilogue& epi,
                    void* stream) override;
@@ -43,7 +47,7 @@ class NetBackend final : public Backend {
   std::unordered_map<int64_t, uint64_t> requests_;  // request id -> engine operation
   std::unordered_map<int64_t, void*> recv_bufs_;    // receive requests: where Wait copies the message
   int64_t next_request_ = 1;
-  NetBuffer scratch_[3];  // grow-only temporaries of the large-message Allreduce
+  NetBuffer scratch_[3];  // grow-only temporaries of the large-message Allreduce and of Scan
 };
 
 // Host backend of a job that spans nodes with the same number of ranks on each: Allreduce is done in three steps -
@@ -67,6 +71,11 @@ class HierBackend final : public Backend {
   // rooted operations: along the root's rail between the nodes, through shared memory inside each node
   void bcast(void* buf, int64_t n, DType dt, int root, void* stream) override;
   void reduce(void* buf, int64_t n, DType dt, ReduceOp op, int root, void* stream) override;
+  // Scan / Exscan: the flat mesh (one fold over all ranks, so 16-bit floats are rounded once)
+  void scan(const void* in, void* out, int64_t n, DType dt, ReduceOp op, bool exclusive, bool reverse,
+            void* stream) override {
+    flat_.scan(in, out, n, dt, op, exclusive, reverse, stream);
+  }
   // slab plans: boxes held by ranks of this node are read through the node's shared memory, the others over the mesh
   void pull(const PullPlan& plan, const void* in, void* out, DType dt, void* stream) override;
   // Reduce_scatter with the same count on every rank: the node first sums, through shared memory, the slices of the

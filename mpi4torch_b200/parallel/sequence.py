@@ -1,6 +1,7 @@
 """Sequence <-> head re-sharding (the Ulysses exchange) as a single
 ``Alltoall(gatheraxis, scatteraxis)``: one kernel instead of the reference's
-4*P blocking collectives (reference csrc/extension.cpp:917-987)."""
+4*P blocking collectives (reference csrc/extension.cpp:917-987), and the
+cumulative sum along a sequence-sharded dimension (one ``Exscan``)."""
 from __future__ import annotations
 
 import torch
@@ -39,3 +40,18 @@ def ulysses_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, comm=No
     out = torch.nn.functional.scaled_dot_product_attention(
         qh.transpose(1, 2), kh.transpose(1, 2), vh.transpose(1, 2), is_causal=causal)  # [B, H/P, S, D]
     return heads_to_sequence(out.transpose(1, 2).contiguous(), 1, 2, c)
+
+
+def distributed_cumsum(x: torch.Tensor, dim: int, comm=None) -> torch.Tensor:
+    """``torch.cumsum`` along a dimension that is sharded by rank, in rank order.
+
+    ``x`` is this rank's shard; every rank passes the same shape apart from ``dim``.  The result is
+    this rank's shard of the cumulative sum of the concatenated tensor: the local cumulative sum plus
+    the sum of all earlier ranks' shards, which one ``Exscan(MPI_SUM)`` of the local totals provides
+    (instead of an ``Allgather`` of the whole tensor).  The gradient comes from autograd: the
+    reverse ``Exscan`` of the gradient totals.
+    """
+    c = m4t.COMM_WORLD if comm is None else comm
+    d = dim if dim >= 0 else dim + x.dim()
+    before = c.Exscan(x.sum(dim=d, keepdim=True), m4t.MPI_SUM)
+    return torch.cumsum(x, d) + before
